@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the packed-genotype hot path (BASELINE.json metric:
 "genotypes/sec in bed_prodVec").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one bed_prodVec (X~ . y, binomial center/scale, all rows, all columns) over the resident synthetic
@@ -22,6 +22,13 @@ same matrix (rank 0), so the timed path is checked against the reference's arith
 `--impl reference` times the reference's CPU implementation of the same call on the host cores: the literal
 C/OpenMP port in oracle/ (the reference needs R + Rcpp + bigstatsr and cannot be built here), all host
 threads, on a bounded column sample of the same synthetic matrix.
+
+`--dump-outputs DIR` writes, after the timed steps, the n-vector the last timed bed_prodVec step returned as
+DIR/<workload>_prodvec.npy (float64; with the default N = 1 run also cfg2_prodvec.npy of the extra leg).  The matrix
+and the vector are generated from fixed seeds, so two builds run with the same arguments can be compared file by file.
+
+bench.py writes nothing into the tree: it uses the CUDA library and the CPU oracle that `python __graft_entry__.py`
+built, and stops if either is missing or older than its sources.
 """
 from __future__ import annotations
 
@@ -35,6 +42,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the tree: the benchmark may run from a read-only checkout
 
 import numpy as np  # noqa: E402
 
@@ -311,6 +319,8 @@ def run_workload(args, wl_key, torch, dist, B, L, rank, world, local, with_cpu, 
         dist.barrier()
     clocks = sampler.stop()
     ms = ev0.elapsed_time(ev1)
+    # the result of the last timed step, copied before the later legs run the product again
+    last_out = out.cpu().numpy() if args.dump_outputs else None
     launches = int(L.bsg_launch_count() - launches0)
     cnt, tot = C.c_int(0), C.c_double(0)
     _lib.check(L.bsg_kernel_time_stats(C.byref(cnt), C.byref(tot)))
@@ -510,6 +520,7 @@ def run_workload(args, wl_key, torch, dist, B, L, rank, world, local, with_cpu, 
                         "with_scaling_reuse: the same after bsg_set_scaling_reuse(1) -- an unchanged scaling (address, "
                         "length, strided sample of the values) is not uploaded again: 8 m bytes up per step"},
         "clocks": clocks, "gpu_launches": launches, "svd": svd_info, "single_copy": single_copy,
+        "outputs": {wl_key + "_prodvec": last_out} if last_out is not None else {},
     }
 
 
@@ -530,7 +541,18 @@ def main():
     ap.add_argument("--nccl", action="store_true", help="N > 1: reduce with torch.distributed / NCCL instead of the library's "
                                                        "own peer-memory communicator (the baseline it is measured against)")
     ap.add_argument("--no-single-copy", action="store_true", help="skip the extra leg timing X.y on the SNP-major copy alone")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm sizes its column sample from a timing, so its inputs vary by run")
+    from bigsnpr_b200 import build
+    from oracle import ref
+
+    for so, old in ((build.OUT, build.stale()), (ref._SO, ref.stale())):
+        if old:
+            raise SystemExit("%s is missing or older than its sources: build first (python __graft_entry__.py)" % so)
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         return run_reference(args, wl)
@@ -554,12 +576,8 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 
     import bigsnpr_b200 as B
-    from bigsnpr_b200 import _lib, build
+    from bigsnpr_b200 import _lib
 
-    if rank == 0:
-        build.build()
-    if world > 1:
-        dist.barrier()
     L = _lib.lib()
     dev = torch.device("cuda", local)
     # a dedicated (non-default) stream: the library enqueues on the stream it is handed, and the CUDA events that time
@@ -584,6 +602,10 @@ def main():
             "parity": res["parity"], "e2e": res["e2e"], "clocks": res["clocks"], "gpu_launches": res["gpu_launches"],
             "svd": res["svd"], "single_copy": res["single_copy"], "extra": extra,
         }
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in {**res["outputs"], **(r2["outputs"] if extra else {})}.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -43,10 +43,14 @@ class OracleError(RuntimeError):
     pass
 
 
+def stale() -> bool:
+    src = os.path.join(_HERE, "bsg_oracle.c")
+    return (not os.path.exists(_SO)) or os.path.getmtime(_SO) < os.path.getmtime(src)
+
+
 def build(force: bool = False) -> str:
     """Compile ``bsg_oracle.c`` (gcc -O2 -fopenmp) if the shared object is missing or stale."""
-    src = os.path.join(_HERE, "bsg_oracle.c")
-    if force or (not os.path.exists(_SO)) or os.path.getmtime(_SO) < os.path.getmtime(src):
+    if force or stale():
         subprocess.check_call(["make", "-s", "-C", _HERE])
     return _SO
 
