@@ -64,6 +64,8 @@ SIGNATURES = {
     "bsg_prod_and_rowsumssq": (C.c_int, [vp, c_int_p, C.c_int, c_int_p, C.c_int, c_dbl_p, c_dbl_p, c_dbl_p, C.c_int,
                                          c_dbl_p, c_dbl_p]),
     "bsg_multlinreg": (C.c_int, [vp, c_int_p, C.c_int, c_int_p, C.c_int, c_dbl_p, C.c_int, c_dbl_p]),
+    "bsg_code256_kind": (C.c_int, [c_dbl_p]),
+    "bsg_impute": (C.c_int, [c_u8_p, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int, c_int_p]),
     "bsg_tcrossprod": (C.c_int, [vp, c_int_p, C.c_int, c_int_p, C.c_int, c_dbl_p, c_dbl_p, c_dbl_p]),
     "bsg_tcrossprod_dev": (C.c_int, [vp, c_int_p, C.c_int, c_int_p, C.c_int, c_dbl_p, c_dbl_p, vp]),
     "bsg_randomsvd": (C.c_int, [vp, c_int_p, C.c_int, c_int_p, C.c_int, c_dbl_p, c_dbl_p, C.c_int, C.c_double,

@@ -35,6 +35,14 @@ NA_INTEGER = -2147483648
 
 LAYOUT_AUTO, LAYOUT_SNP_MAJOR, LAYOUT_SAMPLE_MAJOR = 0, 1, 2
 
+# FBM.code256 code tables (R/bigSNP-class.R:7,13, R/impute.R:9).  A table whose non-NA codes are multiples of 1/100 in
+# [0, 2.54] with one value per multiple, and not only 0 / 1 / 2 (CODE_DOSAGE), is staged as value bytes: bed_prodVec,
+# bed_cprodVec, View and bed_randomSVD then run on the integer tensor pipe.  CODE_012 / CODE_IMPUTE_PRED keep the
+# 2-bit path.
+CODE_012 = np.array([0.0, 1.0, 2.0] + [np.nan] * 253)
+CODE_DOSAGE = np.concatenate([[0.0, 1.0, 2.0, np.nan, 0.0, 1.0, 2.0], 0 + np.arange(201) * 0.01, np.full(48, np.nan)])
+CODE_IMPUTE_PRED = np.array([0.0, 1.0, 2.0, np.nan, 0.0, 1.0, 2.0] + [np.nan] * 249)
+
 
 def _i32(a):
     return np.ascontiguousarray(a, dtype=np.int32)
@@ -732,8 +740,15 @@ def _auto_svd(obj_bed, infos_chr, infos_pos, ind_row, ind_col, fun_scaling, thr_
     say = print if verbose else (lambda *a, **k: None)
     if not (min_mac > 0 and min_maf > 0):
         raise ValueError("You cannot use variants with no variation; set min.mac > 0 and min.maf > 0.")
-    info = bed_MAF(obj_bed, ind_row, ind_col, ncores)
-    nok = (info["mac"] < min_mac) | (info["maf"] < min_maf)
+    try:
+        info = bed_MAF(obj_bed, ind_row, ind_col, ncores)
+        nok = (info["mac"] < min_mac) | (info["maf"] < min_maf)
+    except BsgError:
+        if not fbm:
+            raise
+        # dosage FBM.code256 (no hard-call counts): the reference's own filter, R/autoSVD.R:95-97
+        maf = snp_MAF(obj_bed, ind_row, ind_col, ncores=ncores)
+        nok = maf < max(min_maf, min_mac / (2 * ind_row.size))
     say("Discarding %d variant%s with MAC < %s or MAF < %s." % (nok.sum(), "s" if nok.sum() > 1 else "", min_mac, min_maf))
     ind_keep = ind_col[~nok]
     if thr_r2 is None or np.isnan(thr_r2):
@@ -858,6 +873,47 @@ def bed_projectSelfPCA(obj_svd, obj_bed, ind_row, ind_col=None, ncores=1):
     _assert_lengths(np.arange(v.shape[0]), ind_col)
     XV, x_norm = prod_and_rowSumsSq(obj_bed, ind_row, ind_col, obj_svd["center"], obj_svd["scale"], v)
     return {"obj.svd.ref": obj_svd, "simple_proj": XV, "X_norm": x_norm}
+
+
+def snp_projectSelfPCA(obj_svd, G, ind_row, ind_col=None, ncores=1):
+    """R/bed-projectPCA.R:229-270: bed_projectSelfPCA for the FBM.code256 `G` (a handle from Bed.from_fbm) that the SVD
+    was computed on; the products are prod_and_rowSumsSq2 (src/project-utils.cpp:12-43), served on a centi-dosage
+    handle (CODE_DOSAGE): x = (code256[byte] - center) / scale, a missing value makes its row of XV and X_norm NaN."""
+    return bed_projectSelfPCA(obj_svd, G, ind_row, ind_col, ncores)
+
+
+_IMPUTE_METHODS = ("mode", "mean0", "mean2", "random")
+
+
+def snp_fastImputeSimple(G_bytes, method="mode", code256=CODE_012, seed=None, device=0, ncores=1):
+    """R/impute.R:189-203 (-> src/impute-simple.cpp:10-73): imputes the missing values of the n x m FBM.code256 bytes
+    ``G_bytes`` (numpy uint8, column-major) IN PLACE on the GPU and returns the code table of the result, like
+    ``Gna$copy(code = ...)``: CODE_DOSAGE for "mean2", CODE_IMPUTE_PRED otherwise.  "random" draws from a counter-based
+    generator keyed by (seed, column, row) instead of R's rbinom (``seed`` None: a fresh one).  A column with no
+    non-missing value is left unchanged by "mean0" / "mean2" / "random" (the reference casts NaN to a byte there), with a
+    warning."""
+    import warnings
+
+    if not np.array_equal(np.asarray(code256, dtype=np.float64), CODE_012, equal_nan=True):
+        raise ValueError("identical(Gna$code256, CODE_012) is not TRUE")
+    if isinstance(method, str) and method == "zero":
+        warnings.warn('Using \'method = "zero"\' is deprecated. Using $copy() instead..')
+        return np.array([0.0, 1.0, 2.0, 0.0] + [np.nan] * 252)
+    if method not in _IMPUTE_METHODS:
+        raise ValueError("'arg' should be one of " + ", ".join('"%s"' % m for m in _IMPUTE_METHODS))
+    if not (isinstance(G_bytes, np.ndarray) and G_bytes.dtype == np.uint8 and G_bytes.ndim == 2
+            and G_bytes.flags.f_contiguous and G_bytes.flags.writeable):
+        raise TypeError("G_bytes must be a writeable column-major (n, m) uint8 array: it is imputed in place")
+    n, m = G_bytes.shape
+    k = _IMPUTE_METHODS.index(method) + 1
+    if seed is None:
+        seed = int(np.random.default_rng().integers(0, 2**63))
+    n_all = C.c_int(0)
+    check(lib().bsg_impute(G_bytes.ctypes.data_as(_lib.c_u8_p), int(n), int(m), k, int(seed) & (2**64 - 1), int(device),
+                           C.byref(n_all)))
+    if n_all.value > 0 and k > 1:
+        warnings.warn("%d columns have no non-missing value: left unchanged." % n_all.value)
+    return CODE_DOSAGE.copy() if k == 3 else CODE_IMPUTE_PRED.copy()
 
 
 def multLinReg(obj, ind_row, ind_col, U, ncores=1):

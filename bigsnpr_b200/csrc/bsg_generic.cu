@@ -155,7 +155,7 @@ static int grid_warps(long long items) { return (int)std::max<long long>(1, std:
 int generic_colstats(bsg_bed *h, const int *d_row, int nr, const int *d_col, int nc, double *d_sumX, double *d_denoX,
                      cudaStream_t s) {
   if (nc <= 0) return BSG_OK;
-  gen::k_colstats<<<gen::grid_warps(nc), 256, 0, s>>>(h->raw, h->n, h->d_code, d_row, nr, d_col, nc, d_sumX, d_denoX);
+  gen::k_colstats<<<gen::grid_warps(nc), 256, 0, s>>>(h->raw, h->raw_stride, h->d_code, d_row, nr, d_col, nc, d_sumX, d_denoX);
   count_launch();
   BSG_CUDA(cudaGetLastError());
   return BSG_OK;
@@ -168,11 +168,11 @@ int generic_pairs(bsg_bed *h, const int *d_row, int nr, const int *d_col, int nc
   const int grid = gen::grid_warps(total);
   const double *c3 = h->d_code + 256;
   if (kind == 0)
-    gen::k_pairs<0><<<grid, 256, 0, s>>>(h->raw, h->n, c3, h->d_code, d_row, nr, d_col, nc, d_wlen, d_boff, total, d_thr, d_band, d_keep, d_sumX, d_denoX, thr_r2);
+    gen::k_pairs<0><<<grid, 256, 0, s>>>(h->raw, h->raw_stride, c3, h->d_code, d_row, nr, d_col, nc, d_wlen, d_boff, total, d_thr, d_band, d_keep, d_sumX, d_denoX, thr_r2);
   else if (kind == 1)
-    gen::k_pairs<1><<<grid, 256, 0, s>>>(h->raw, h->n, c3, h->d_code, d_row, nr, d_col, nc, d_wlen, d_boff, total, d_thr, d_band, d_keep, d_sumX, d_denoX, thr_r2);
+    gen::k_pairs<1><<<grid, 256, 0, s>>>(h->raw, h->raw_stride, c3, h->d_code, d_row, nr, d_col, nc, d_wlen, d_boff, total, d_thr, d_band, d_keep, d_sumX, d_denoX, thr_r2);
   else
-    gen::k_pairs<3><<<grid, 256, 0, s>>>(h->raw, h->n, c3, h->d_code, d_row, nr, d_col, nc, d_wlen, d_boff, total, d_thr, d_band, d_keep, d_sumX, d_denoX, thr_r2);
+    gen::k_pairs<3><<<grid, 256, 0, s>>>(h->raw, h->raw_stride, c3, h->d_code, d_row, nr, d_col, nc, d_wlen, d_boff, total, d_thr, d_band, d_keep, d_sumX, d_denoX, thr_r2);
   count_launch();
   BSG_CUDA(cudaGetLastError());
   return BSG_OK;
@@ -181,7 +181,7 @@ int generic_pairs(bsg_bed *h, const int *d_row, int nr, const int *d_col, int nc
 int generic_multlinreg(bsg_bed *h, const int *d_row, int nr, const int *d_col, int nc, const double *d_U, int K,
                        double *d_out, cudaStream_t s) {
   if (nc <= 0 || K <= 0) return BSG_OK;
-  gen::k_multlinreg<<<gen::grid_warps(nc), 256, 0, s>>>(h->raw, h->n, h->d_code + 256, d_row, nr, d_col, nc, d_U, K, d_out);
+  gen::k_multlinreg<<<gen::grid_warps(nc), 256, 0, s>>>(h->raw, h->raw_stride, h->d_code + 256, d_row, nr, d_col, nc, d_U, K, d_out);
   count_launch();
   BSG_CUDA(cudaGetLastError());
   return BSG_OK;

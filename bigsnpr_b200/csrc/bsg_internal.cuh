@@ -95,8 +95,13 @@ struct bsg_bed {
   int na_ell = 0;            // 0 not tried yet, 1 resident, -1 not used (rate too high, no memory, disabled)
   double code256[256];       // FBM handles: value of each raw byte code (bigstatsr code256)
   int fbm_generic = 0;       // FBM whose codes are not {0,1,2,NA} (dosages ...): served by the fp64 kernels of bsg_generic.cu
-  uint8_t *raw = nullptr;    // generic FBM: the n x m code bytes, column-major, as in the .bk file
-  double *d_code = nullptr;  // generic FBM: code256 on the device [0,256) and the same with NA -> 3 [256,512)
+  uint8_t *raw = nullptr;    // generic FBM: the n x m code bytes, column-major, line j at raw + j * raw_stride
+  int64_t raw_stride = 0;    // n, or round_up(n, 512) with zero padding for a centi-dosage handle
+  double *d_code = nullptr;  // generic FBM: byte value on the device [0,256) and the same with NA -> 3 [256,512)
+  // centi-dosage FBM (every code a multiple of 1/100 in [0, 2.54], bsg_core.cu): raw holds VALUE bytes rint(100 x), 255 =
+  // missing, and d_code is indexed by value byte; the matvecs run on the integer tensor pipe (bsg_pmv8.cu)
+  int dosage = 0;
+  std::vector<int> na_line;  // centi-dosage: missing values per SNP line over all n samples
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t copy_stream = nullptr;  // created on first use: host -> device uploads that run under the kernels of `stream`
@@ -185,6 +190,22 @@ int generic_pairs(bsg_bed *h, const int *d_row, int nr, const int *d_col, int nc
 int generic_multlinreg(bsg_bed *h, const int *d_row, int nr, const int *d_col, int nc, const double *d_U, int K,
                        double *d_out, cudaStream_t s);
 
+// ---- bsg_pmv8.cu: centi-dosage handles (value bytes) ----------------------------------------------------------------
+// code table -> value byte per code (255 = NA); false when the table is not centi-dosage (see bsg_open_fbm256)
+bool dosage_value_bytes(const double *code256, uint8_t vbyte[256]);
+// value bytes with a zero-padded line stride + missing values per line, from the n x m code bytes on the device
+int dosage_stage(bsg_bed *h, const uint8_t *d_codes, const uint8_t *d_vbyte);
+// Xt.y on the value bytes: lines = SNP columns, contraction over all n samples (pmv::Args: dig1 = k_prep2 / k_digits
+// layout, part zeroed here); the NA plane is never used
+namespace pmv { struct Args; }
+int run_pmv8(bsg_view *v, const uint8_t *dig, pmv::Args *out, cudaStream_t s);
+// view scaling of a centi-dosage handle: d_center, d_scale (uploaded as c, s) -> 100 c, 100 s
+int dosage_view_scaling(bsg_view *v, cudaStream_t s);
+// host-vector forms: out[t] = NaN for every output entry whose row / column meets a selected missing value
+int dosage_mark_na(bsg_view *v, bool cprod, double *d_out, cudaStream_t s);
+// prod_and_rowSumsSq2 on a centi-dosage view (host V / XV / rowSumsSq, synchronous)
+int dosage_prod_and_rowsumssq(bsg_view *v, const double *V, int K, double *XV, double *rowSumsSq);
+
 // ---- bsg_gramt.cu: integer Gram tiles fed by TMA, 2-CTA tcgen05 MMAs (GRM and windowed correlations) ----------
 namespace gram { struct Tile; }
 bool gramt_enabled();  // BSG_GRAM_TMA=0 selects the round-1 kernels (in-kernel expansion) for cross-checks
@@ -227,11 +248,14 @@ struct bsg_view {
   int nr = 0, nc = 0;
   int row_identity = 1, col_identity = 1;
   int row_maxmult = 1, col_maxmult = 1;
-  int has_scaling = 0;       // center/scale given (else 0 / 1)
+  int has_scaling = 0;       // center/scale given (else 0 / 1); always 1 on a centi-dosage handle
+  int any_na = 0;            // centi-dosage: a selected SNP column holds a missing value
+  int *d_na_pos = nullptr;   // centi-dosage: positions (in ind_col) of the selected columns holding a missing value
+  int n_na_pos = 0;
   // device arrays (owned)
   int *d_row = nullptr;      // [nr] 0-based rows (null if identity)
   int *d_col = nullptr;      // [nc] 0-based cols (null if identity)
-  double *d_center = nullptr, *d_scale = nullptr;  // [nc] (null if !has_scaling)
+  double *d_center = nullptr, *d_scale = nullptr;  // [nc] (null if !has_scaling); 100 c, 100 s on a centi-dosage handle
   // prodvec over copy B: distinct rows to compute and the gather map back to ind_row order
   int *d_rows_unique = nullptr;  // [nru] sorted distinct rows (null if identity)
   int *d_row_gather = nullptr;   // [nr] position of each requested row in d_rows_unique

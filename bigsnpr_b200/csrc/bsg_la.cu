@@ -453,6 +453,9 @@ int lanczos_svd(std::vector<SvdShard> &sh, const int *ind_row, int nr, int ncol_
     if (sh[g].center && sh[g].scale) {
       memcpy(rep[g].cen.data(), sh[g].center, (size_t)nc * sizeof(double));
       memcpy(rep[g].sca.data(), sh[g].scale, (size_t)nc * sizeof(double));
+    } else if (h->dosage) {
+      return fail(BSG_ERR_ARG, "bed_scaleBinom needs hard calls: pass center and scale for a dosage FBM.code256 "
+                               "(snp_scaleBinom, or the mean and sd of each column).");
     } else if (nc > 0) {
       std::vector<double> sumX(nc), denoX(nc);
       std::vector<int> nona(nc);

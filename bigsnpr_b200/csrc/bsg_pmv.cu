@@ -47,80 +47,6 @@
 namespace bsg {
 namespace pmv {
 
-constexpr int SEG = 128;              // bytes per line per stage = 512 codes
-constexpr int CODES = 512;            // codes per line per stage
-constexpr int DIG = 4096;             // digit bytes per stage per plane (512 codes x 8 slices)
-constexpr int STAGES = 6;
-constexpr int STAGE_BYTES = 2 * DIG;  // raw-plane digits + NA-plane digits
-constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 128;
-// Variants <CW consumer warps, R chunks of register ring per warp>; lines per work item = 32 * CW.
-// Register file: (CW + 1) warps share 4 SMSPs of 16 K registers -> cap 255 regs for 8 warps, 168 for 9..12.
-constexpr int MAX_CHUNKS_PER_ITEM = 512;  // 262144 codes: |acc16| <= 262144*48*128 < 2^31
-
-struct Args {
-  const uint8_t *P;
-  int64_t stride;
-  const int *lines;      // physical line per logical line (null = identity)
-  int nlines;
-  int nlines_pad;        // multiple of the group size (32 * consumer warps)
-  int nchunks;           // 128-byte chunks per line
-  int chunks_per_split;
-  int ksplit;
-  const uint8_t *dig1;   // [nchunks][DIG]
-  const uint8_t *dig2;   // NA-plane digits (null = same as dig1)
-  const uint8_t *na_flags;  // per physical line (null = assume missing values anywhere)
-  int use_na;            // 0: matrix has no missing value, skip the NA plane
-  long long *part;       // [nlines_pad][16] zeroed accumulators: 8 raw-plane slices, 8 NA-plane slices
-};
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(bar),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ void mma_u8s8(int (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
-                                         uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+r"(d[0]), "+r"(d[1]), "+r"(d[2]), "+r"(d[3])
-      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint4 lds128(uint32_t addr) {
-  uint4 v;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
-  return v;
-}
-
-__device__ __forceinline__ uint4 ldg_stream(const uint8_t *p) {
-  uint4 v;
-  asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-               : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-               : "l"(p));
-  return v;
-}
-
 // Fragment bytes of one lane for one 16-line sub-tile and one 128-byte chunk: lines g (a*) and g+8 (b*),
 // bytes [16q, 16q+16) (lo) and [64+16q, 64+16q+16) (hi) of the chunk.
 struct Slot {
@@ -820,7 +746,7 @@ using namespace pmv;
 constexpr int TLINES = 32, TBYTES = 512, TWARPS = 8, TSTAGES = 6;
 constexpr int WSTAGE_BYTES = TLINES * 64;                  // one warp's strip of a step: 32 lines x 64 B
 constexpr int TSMEM = TWARPS * TSTAGES * WSTAGE_BYTES;     // 96 KB -> 2 CTAs per SM
-constexpr int MAX_LINES_PER_ITEM = 1 << 16;                // 64 x 3 x 128 x 2^16 < 2^31
+constexpr int MAX_LINES_PER_ITEM = 1 << 16;                // 64 x 3 x 128 x 2^16 < 2^31; value bytes: 254 x 128 x 2^16 < 2^31
 
 struct TArgs {
   const uint8_t *P;
@@ -840,13 +766,9 @@ __device__ __forceinline__ uint32_t lds32(uint32_t addr) {
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
   return v;
 }
-__device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
-  uint32_t r;
-  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(sel));
-  return r;
-}
-
-template <int PLANE, bool LINES>
+// BYTES: the lines hold one value byte per sample (centi-dosage FBM handles, bsg_pmv8.cu) instead of four 2-bit codes; a
+// transposed word is then directly the A fragment of ONE IMMA (4 lines x 1 sample), no field masks, no 4^c to undo.
+template <int PLANE, bool LINES, bool BYTES = false>
 __global__ void __launch_bounds__(TWARPS * 32, 2) k_pmvT(const TArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, q = lane & 3;
@@ -935,6 +857,10 @@ __global__ void __launch_bounds__(TWARPS * 32, 2) k_pmvT(const TArgs a) {
         wc2 = (wc2 >> 1) & 0x55555555u;
         wd = (wd >> 1) & 0x55555555u;
       }
+      if (BYTES) {
+        mma_u8s8(acc[j][0], wa, wb, wc2, wd, b0, b1);
+        continue;
+      }
       // field c of every byte enters as 4^c x code (exact, undone in the epilogue): no shifts in the loop
       mma_u8s8(acc[j][0], wa & 0x03030303u, wb & 0x03030303u, wc2 & 0x03030303u, wd & 0x03030303u, b0, b1);
       mma_u8s8(acc[j][1], wa & 0x0C0C0C0Cu, wb & 0x0C0C0C0Cu, wc2 & 0x0C0C0C0Cu, wd & 0x0C0C0C0Cu, b0, b1);
@@ -994,10 +920,10 @@ __global__ void __launch_bounds__(TWARPS * 32, 2) k_pmvT(const TArgs a) {
 #pragma unroll
   for (int j = 0; j < 4; j++)
 #pragma unroll
-    for (int c = 0; c < 4; c++)
+    for (int c = 0; c < (BYTES ? 1 : 4); c++)
 #pragma unroll
       for (int sl = 0; sl < 2; sl++) {
-        const int64_t sample = 4 * (byte0 + 4 * (8 * sl + g) + j) + c;
+        const int64_t sample = BYTES ? byte0 + 4 * (8 * sl + g) + j : 4 * (byte0 + 4 * (8 * sl + g) + j) + c;
         if (sample < a.n) {
           unsigned long long *dst = reinterpret_cast<unsigned long long *>(a.part) + sample * 16 + (PLANE ? 8 : 0) + 2 * q;
           long long v0 = acc[j][c][2 * sl], v1 = acc[j][c][2 * sl + 1];
@@ -1399,7 +1325,7 @@ int bsg_view_create(bsg_bed *h, const int *ind_row, int nr, const int *ind_col, 
                     const double *scale, bsg_view **out) {
   if (!h || !out) return fail(BSG_ERR_ARG, "null argument");
   *out = nullptr;
-  BSG_PACKED_ONLY(h, "The packed matrix-vector engine");
+  if (!h->dosage) BSG_PACKED_ONLY(h, "The packed matrix-vector engine");
   BSG_TRY(bind_device(h));
   if (!ind_row) nr = h->n;
   if (!ind_col) nc = h->m;
@@ -1418,6 +1344,19 @@ int bsg_view_create(bsg_bed *h, const int *ind_row, int nr, const int *ind_col, 
     bool ident = true;
     for (int j = 0; j < nc && ident; j++) ident = center[j] == 0.0 && scale[j] == 1.0;
     if (ident) v->has_scaling = 0;
+  }
+  // value bytes are 100 x the dosage: the scaling is always applied, as (100 c, 100 s), default (0, 100)
+  std::vector<double> dos_c, dos_s;
+  if (h->dosage) {
+    v->has_scaling = 1;
+    dos_c.assign(std::max(nc, 1), 0.0);
+    dos_s.assign(std::max(nc, 1), 1.0);
+    if (center) {
+      std::copy(center, center + nc, dos_c.begin());
+      std::copy(scale, scale + nc, dos_s.begin());
+    }
+    center = dos_c.data();
+    scale = dos_s.data();
   }
   cudaStream_t s = h->stream;
   int rc = BSG_OK;
@@ -1460,6 +1399,15 @@ int bsg_view_create(bsg_bed *h, const int *ind_row, int nr, const int *ind_col, 
     rc = dev_copy((void **)&v->d_center, center, (size_t)nc * sizeof(double), s);
     if (!rc) rc = dev_copy((void **)&v->d_scale, scale, (size_t)nc * sizeof(double), s);
   }
+  std::vector<int> na_pos;
+  if (!rc && h->dosage) {
+    rc = dosage_view_scaling(v, s);
+    for (int j = 0; j < nc && !rc; j++)
+      if (h->na_line[v->col_identity ? j : zc[j]] > 0) na_pos.push_back(j);
+    v->n_na_pos = (int)na_pos.size();
+    v->any_na = v->n_na_pos > 0;
+    if (!rc && v->any_na) rc = dev_copy((void **)&v->d_na_pos, na_pos.data(), na_pos.size() * sizeof(int), s);
+  }
   if (!rc) rc = v->s_scal.ensure(2 * sizeof(pmv::Scal));  // the second block serves the two-vectors-per-pass mode
   cudaError_t e = cudaStreamSynchronize(s);  // host vectors go out of scope
   if (!rc && e != cudaSuccess) rc = cuda_fail(e, "view upload");
@@ -1475,7 +1423,7 @@ void bsg_view_destroy(bsg_view *v) {
   if (!v) return;
   cudaSetDevice(v->h->device);
   cudaStreamSynchronize(v->h->stream);
-  void *ptrs[] = {v->d_row, v->d_col, v->d_center, v->d_scale, v->d_rows_unique, v->d_row_gather};
+  void *ptrs[] = {v->d_row, v->d_col, v->d_center, v->d_scale, v->d_rows_unique, v->d_row_gather, v->d_na_pos};
   for (void *p : ptrs)
     if (p) cudaFree(p);
   DevBuf *bufs[] = {&v->s_vec0, &v->s_vec1, &v->s_vec2, &v->s_q0, &v->s_q1, &v->s_dig1,
@@ -1484,25 +1432,37 @@ void bsg_view_destroy(bsg_view *v) {
   delete v;
 }
 
-// t(X~) x : lines = SNP columns of copy A, contraction over samples
-int bsg_view_cprodvec_dev(bsg_view *v, const double *x_dev, double *out_dev, void *stream) {
+}  // extern "C"
+
+__global__ void k_fill(double *x, int len, double v) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < len; i += gridDim.x * blockDim.x) x[i] = v;
+}
+
+// device-vector forms on a centi-dosage view with a selected missing value: the whole output is NaN (bsgpu.h)
+static int dosage_na_fill(bsg_view *v, double *out_dev, int len, cudaStream_t s) {
+  if (!v->h->dosage || !v->any_na || len == 0) return BSG_OK;
+  k_fill<<<std::min(1184, (len + 255) / 256), 256, 0, s>>>(out_dev, len, nan(""));
+  count_launch();
+  BSG_CUDA(cudaGetLastError());
+  return BSG_OK;
+}
+
+// t(X~) x : lines = SNP columns of copy A (value bytes on a centi-dosage handle), contraction over samples
+static int cprodvec_dev(bsg_view *v, const double *x_dev, double *out_dev, cudaStream_t s) {
   if (!v || !x_dev || !out_dev) return fail(BSG_ERR_ARG, "null argument");
   bsg_bed *h = v->h;
   BSG_TRY(bind_device(h));
-  // NULL = the legacy default stream (what the header documents and what torch's default stream is): work is then
-  // ordered with the caller's kernels and collectives, not on the handle's private non-blocking stream
-  cudaStream_t s = stream ? (cudaStream_t)stream : cudaStreamLegacy;
   if (v->nc == 0) return BSG_OK;
   using namespace pmv;
   Scal *sc = v->s_scal.as<Scal>();
   const int n = h->n;
-  int nchunks = (int)(h->strideA / SEG);
+  int nchunks = (int)((h->dosage ? h->raw_stride : h->strideA * 4) / CODES);
   BSG_TRY(v->s_q0.ensure((size_t)n * sizeof(long long)));
   BSG_TRY(v->s_dig1.ensure((size_t)nchunks * DIG));
   long long *Q = v->s_q0.as<long long>();
   const int hb = hb_bits(v->row_maxmult);
   // few missing values: the kernel runs in its no-missing mode and the N plane comes from the per-SNP lists
-  const bool lists = h->has_na && na_ell_ready(h);
+  const bool lists = !h->dosage && h->has_na && na_ell_ready(h);
   if (v->row_identity) {
     // direct path: memset + 2 kernels
     BSG_CUDA(cudaMemsetAsync(sc, 0, sizeof(Scal), s));
@@ -1522,14 +1482,27 @@ int bsg_view_cprodvec_dev(bsg_view *v, const double *x_dev, double *out_dev, voi
     count_launch(6);
   }
   Args a;
-  BSG_TRY(run_pmv(v, h->A, h->strideA, n, v->d_col, v->nc, v->s_dig1.as<uint8_t>(), nullptr, h->naA,
-                  lists ? 0 : h->has_na, &a, s));
+  if (h->dosage)
+    BSG_TRY(run_pmv8(v, v->s_dig1.as<uint8_t>(), &a, s));
+  else
+    BSG_TRY(run_pmv(v, h->A, h->strideA, n, v->d_col, v->nc, v->s_dig1.as<uint8_t>(), nullptr, h->naA,
+                    lists ? 0 : h->has_na, &a, s));
   if (lists) BSG_TRY(na_ell_correction(h, 1, v->d_col, v->nc, Q, a.part, s));
   k_finish_cprod<<<(v->nc + 255) / 256, 256, 0, s>>>(a.part, a.ksplit, a.nlines_pad, v->nc, sc, v->d_center, v->d_scale,
-                                                      h->has_na, out_dev);
+                                                      h->has_na && !h->dosage, out_dev);
   count_launch();
   BSG_CUDA(cudaGetLastError());
   return BSG_OK;
+}
+
+extern "C" {
+
+int bsg_view_cprodvec_dev(bsg_view *v, const double *x_dev, double *out_dev, void *stream) {
+  // NULL = the legacy default stream (what the header documents and what torch's default stream is): work is then
+  // ordered with the caller's kernels and collectives, not on the handle's private non-blocking stream
+  cudaStream_t s = stream ? (cudaStream_t)stream : cudaStreamLegacy;
+  BSG_TRY(cprodvec_dev(v, x_dev, out_dev, s));
+  return dosage_na_fill(v, out_dev, v->nc, s);
 }
 
 // Launcher of k_pmvT: raw plane with `dig_raw`, then (plane != 0) the flag plane (1 = missing value, 2 = high bit)
@@ -1547,13 +1520,14 @@ static int run_pmvT(bsg_view *v, const uint8_t *dig_raw, int plane, const uint8_
   BSG_CUDA(cudaMemsetAsync(part, 0, (size_t)n * 16 * sizeof(long long), s));
   if (nc == 0 || n == 0) return BSG_OK;
   TArgs a;
-  a.P = h->A;
-  a.stride = h->strideA;
+  a.P = h->dosage ? h->raw : h->A;
+  a.stride = h->dosage ? h->raw_stride : h->strideA;
   a.lines = v->d_col;
   a.nlines = nc;
   a.n = n;
   a.part = part;
-  const int64_t nbytes = ((int64_t)n + 3) / 4;
+  if (h->dosage && plane) return fail(BSG_ERR_ARG, "value-byte lines have no flag plane");
+  const int64_t nbytes = h->dosage ? (int64_t)n : ((int64_t)n + 3) / 4;
   a.nblocks = (int)((nbytes + TBYTES - 1) / TBYTES);
   int nsm = 148;
   cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, h->device);
@@ -1600,6 +1574,8 @@ static int run_pmvT(bsg_view *v, const uint8_t *dig_raw, int plane, const uint8_
   if (!(attr_done >> (h->device & 31) & 1u)) {
     BSG_CUDA(cudaFuncSetAttribute(k_pmvT<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TSMEM));
     BSG_CUDA(cudaFuncSetAttribute(k_pmvT<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TSMEM));
+    BSG_CUDA(cudaFuncSetAttribute(k_pmvT<0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TSMEM));
+    BSG_CUDA(cudaFuncSetAttribute(k_pmvT<0, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TSMEM));
     BSG_CUDA(cudaFuncSetAttribute(k_pmvT2<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2SMEM));
     BSG_CUDA(cudaFuncSetAttribute(k_pmvT2<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2SMEM));
     BSG_CUDA(cudaFuncSetAttribute(k_pmvT2<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, T2SMEM));
@@ -1612,7 +1588,11 @@ static int run_pmvT(bsg_view *v, const uint8_t *dig_raw, int plane, const uint8_
   if (g_timing) cudaEventRecord(g_ev0[g_ev_n % EV_POOL], s);
   if (!plane) {
     const int grid = a.nblocks * a.ksplit;
-    if (lines)
+    if (h->dosage && lines)
+      k_pmvT<0, true, true><<<grid, thr, TSMEM, s>>>(a);
+    else if (h->dosage)
+      k_pmvT<0, false, true><<<grid, thr, TSMEM, s>>>(a);
+    else if (lines)
       k_pmvT<0, true><<<grid, thr, TSMEM, s>>>(a);
     else
       k_pmvT<0, false><<<grid, thr, TSMEM, s>>>(a);
@@ -1673,8 +1653,9 @@ static int prodvec_T(bsg_view *v, const double *x_dev, double *out_dev, cudaStre
   Scal *sc = v->s_scal.as<Scal>();
   const int n = h->n, nc = v->nc;
   const int mode = v->has_scaling ? 1 : 0;
-  const bool lists = h->has_na && na_ell_ready(h);  // few missing values: per-sample lists instead of the flag plane
-  const bool two = v->has_scaling && h->has_na && !lists;
+  const bool na = h->has_na && !h->dosage;  // value bytes: missing values are marked after the product (bsg_pmv8.cu)
+  const bool lists = na && na_ell_ready(h);  // few missing values: per-sample lists instead of the flag plane
+  const bool two = v->has_scaling && na && !lists;
   long long *qna = nullptr;
   if (lists) {  // the missing-value vector ((c - 3) z with scaling, else y) by physical SNP
     BSG_TRY(v->s_q1.ensure((size_t)h->m * sizeof(long long)));
@@ -1683,7 +1664,7 @@ static int prodvec_T(bsg_view *v, const double *x_dev, double *out_dev, cudaStre
   }
   BSG_TRY(prep_T(v, mode, x_dev, v->d_center, v->d_scale, two, s, qna, v->has_scaling ? 1 : 0));  // incl. the partials of C
   long long *part = nullptr;
-  BSG_TRY(run_pmvT(v, v->s_dig1.as<uint8_t>(), (h->has_na && !lists) ? 1 : 0,
+  BSG_TRY(run_pmvT(v, v->s_dig1.as<uint8_t>(), (na && !lists) ? 1 : 0,
                    two ? v->s_dig2.as<uint8_t>() : v->s_dig1.as<uint8_t>(), &part, s));
   if (lists) BSG_TRY(na_ell_correction(h, 0, nullptr, n, qna, part, s));
   double *full = out_dev;
@@ -1694,7 +1675,7 @@ static int prodvec_T(bsg_view *v, const double *x_dev, double *out_dev, cudaStre
   if (comm && v->row_identity)  // epilogue fused with the sum over the column shards (NVLink peer memory, bsg_comm.cu)
     return comm_finish_prod_allreduce(comm, part, n, sc, v->has_scaling, h->has_na, out_dev, s);
   if (n > 0) {
-    k_finish_prod<<<(n + 255) / 256, 256, 0, s>>>(part, 1, n, n, sc, v->has_scaling, h->has_na, full);
+    k_finish_prod<<<(n + 255) / 256, 256, 0, s>>>(part, 1, n, n, sc, v->has_scaling, na, full);
     count_launch();
   }
   if (!v->row_identity && v->nr > 0) {
@@ -1763,7 +1744,7 @@ static bool use_T(const bsg_bed *h) {
   }
   // with missing values the fused SNP-major kernel (k_pmvT2, 1.68 ms at cfg2) is ahead of the sample-major
   // kernel's NA mode (1.81 ms); without, the sample-major kernel keeps a 1-3 % edge when its copy is resident
-  return !h->B || g_force_t == 1 || h->has_na;
+  return !h->B || g_force_t == 1 || h->has_na || h->dosage;
 }
 
 }  // extern "C"
@@ -1775,6 +1756,7 @@ int bsg::view_prodvec_comm(bsg_view *v, const double *x_dev, double *out_dev, cu
   bsg_bed *h = v->h;
   BSG_TRY(bind_device(h));
   if (v->nr == 0) return BSG_OK;
+  if (h->dosage && comm) return fail(BSG_ERR_ARG, "centi-dosage handles have no column-sharded form");
   if (use_T(h)) return prodvec_T(v, x_dev, out_dev, s, comm);  // transposing kernel over the SNP-major copy
   using namespace pmv;
   Scal *sc = v->s_scal.as<Scal>();
@@ -1838,7 +1820,9 @@ extern "C" {
 int bsg_view_prodvec_dev(bsg_view *v, const double *x_dev, double *out_dev, void *stream) {
   // NULL = the legacy default stream (what the header documents and what torch's default stream is): work is then
   // ordered with the caller's kernels and collectives, not on the handle's private non-blocking stream
-  return view_prodvec_comm(v, x_dev, out_dev, stream ? (cudaStream_t)stream : cudaStreamLegacy, nullptr);
+  cudaStream_t s = stream ? (cudaStream_t)stream : cudaStreamLegacy;
+  BSG_TRY(view_prodvec_comm(v, x_dev, out_dev, s, nullptr));
+  return v->nr ? dosage_na_fill(v, out_dev, v->nr, s) : BSG_OK;
 }
 
 // host-vector front ends: H2D of x, the product, D2H of the result; non-finite input falls back to the
@@ -1853,13 +1837,14 @@ static int view_host_call(bsg_view *v, const double *x, double *out, bool cprod)
   BSG_TRY(v->s_vec1.ensure((size_t)std::max(nout, 1) * sizeof(double)));
   double *dx = v->s_vec0.as<double>(), *dout = v->s_vec1.as<double>();
   BSG_CUDA(cudaMemcpyAsync(dx, x, (size_t)nin * sizeof(double), cudaMemcpyHostToDevice, s));
-  BSG_TRY(cprod ? bsg_view_cprodvec_dev(v, dx, dout, s) : bsg_view_prodvec_dev(v, dx, dout, s));
+  BSG_TRY(cprod ? cprodvec_dev(v, dx, dout, s) : view_prodvec_comm(v, dx, dout, s, nullptr));
+  if (h->dosage) BSG_TRY(dosage_mark_na(v, cprod, dout, s));
   int bad = 0;
   if (nout > 0)  // every product path (copy A or copy B) raises the flag on non-finite input
     BSG_CUDA(cudaMemcpyAsync(&bad, &v->s_scal.as<pmv::Scal>()->nonfinite, sizeof(int), cudaMemcpyDeviceToHost, s));
   BSG_CUDA(cudaMemcpyAsync(out, dout, (size_t)nout * sizeof(double), cudaMemcpyDeviceToHost, s));
   BSG_CUDA(cudaStreamSynchronize(s));
-  if (bad) {
+  if (bad && !h->dosage) {  // (a centi-dosage handle keeps the finish kernels' all-NaN output)
     BSG_TRY(cprod ? simple_cprodvec(h, v->d_row, v->nr, v->d_col, v->nc, v->d_center, v->d_scale, dx, dout, s)
                   : simple_prodvec(h, v->d_row, v->nr, v->d_col, v->nc, v->d_center, v->d_scale, dx, dout, s));
     BSG_CUDA(cudaMemcpyAsync(out, dout, (size_t)nout * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -1937,6 +1922,7 @@ static int cached_view(bsg_bed *h, const int *ind_row, int nr, const int *ind_co
     if (!same) {
       BSG_CUDA(cudaMemcpyAsync(h->cv->d_center, center, (size_t)nc * sizeof(double), cudaMemcpyHostToDevice, h->stream));
       BSG_CUDA(cudaMemcpyAsync(h->cv->d_scale, scale, (size_t)nc * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+      if (h->dosage) BSG_TRY(dosage_view_scaling(h->cv, h->stream));
       h->cv_center_ptr = center;
       h->cv_scale_ptr = scale;
       h->cv_scal_sample.swap(smp);
@@ -2198,9 +2184,6 @@ struct ProjScratch {
 // bed_row_counts_cpp (src/bed-fun.cpp:72-98) from three linear functionals of the all-ones vector over the selected
 // columns: R = c1 + 2 c2 + 3 c3 (raw codes), N = c3 (missing flag), H = c2 + c3 (high bit).  Sums of exactly
 // representable integers: the counts are exact.
-__global__ void k_fill(double *x, int len, double v) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < len; i += gridDim.x * blockDim.x) x[i] = v;
-}
 __global__ void k_counts_from_planes(int nr, int nc, const double *__restrict__ R, const double *__restrict__ N,
                                      const double *__restrict__ H, int32_t *__restrict__ out4) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -2247,8 +2230,10 @@ int bsg_prod_and_rowsumssq(bsg_bed *h, const int *ind_row, int nr, const int *in
   if (!h || !XV || !rowSumsSq || (!V && K > 0)) return fail(BSG_ERR_ARG, "null argument");
   if (!center || !scale) return fail(BSG_ERR_DIM, "Incompatibility between dimensions.");
   if (K < 0) return fail(BSG_ERR_ARG, "negative length");
+  if (!h->dosage) BSG_PACKED_ONLY(h, "prod_and_rowSumsSq");
   bsg_view *v = nullptr;
   BSG_TRY(cached_view(h, ind_row, nr, ind_col, nc, center, scale, &v));
+  if (h->dosage) return dosage_prod_and_rowsumssq(v, V, K, XV, rowSumsSq);  // prod_and_rowSumsSq2 (bsg_pmv8.cu)
   nr = v->nr;
   nc = v->nc;
   cudaStream_t s = h->stream;

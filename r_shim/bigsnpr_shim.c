@@ -13,6 +13,7 @@
  */
 #include <R.h>
 #include <Rinternals.h>
+#include <R_ext/Random.h>
 #include <R_ext/Rdynload.h>
 
 #include <fcntl.h>
@@ -330,6 +331,43 @@ SEXP _bigsnpr_prod_and_rowSumsSq(SEXP obj_bed, SEXP ind_row, SEXP ind_col, SEXP 
   return res;
 }
 
+/* _bigsnpr_prod_and_rowSumsSq2: src/project-utils.cpp:12-43 (6 arguments; snp_projectSelfPCA, R/bed-projectPCA.R:229-270)
+ * -> list(XV, rowSumsSq) on an FBM.code256 environment (centi-dosage codes: include/bsgpu.h) */
+SEXP _bigsnpr_prod_and_rowSumsSq2(SEXP BM, SEXP ind_row, SEXP ind_col, SEXP center, SEXP scale, SEXP V) {
+  bsg_bed *h = fbm_handle_of(BM);
+  int nr = LENGTH(ind_row), nc = LENGTH(ind_col), K = Rf_ncols(V);
+  if (LENGTH(center) != nc || LENGTH(scale) != nc || Rf_nrows(V) != nc) Rf_error("Incompatibility between dimensions.");
+  SEXP XV = PROTECT(Rf_allocMatrix(REALSXP, nr, K)), rss = PROTECT(Rf_allocVector(REALSXP, nr));
+  chk(bsg_prod_and_rowsumssq(h, INTEGER(ind_row), nr, INTEGER(ind_col), nc, REAL(center), REAL(scale), REAL(V), K, REAL(XV),
+                             REAL(rss)));
+  for (R_xlen_t i = 0; i < XLENGTH(XV); i++)
+    if (ISNAN(REAL(XV)[i])) REAL(XV)[i] = NA_REAL; /* a missing dosage: NA_real_ like bigstatsr's accessor */
+  for (int i = 0; i < nr; i++)
+    if (ISNAN(REAL(rss)[i])) REAL(rss)[i] = NA_REAL;
+  SEXP res = PROTECT(Rf_allocVector(VECSXP, 2));
+  SET_VECTOR_ELT(res, 0, XV);
+  SET_VECTOR_ELT(res, 1, rss);
+  UNPROTECT(3);
+  return res;
+}
+
+/* _bigsnpr_impute: src/impute-simple.cpp:10-73 (3 arguments; snp_fastImputeSimple, R/impute.R:189-203).  The bytes of the
+ * FBM.code256 are imputed in place through a shared writable mapping of its backing file; the seed of the random method
+ * comes from R's RNG (set.seed reproduces it).  A staged copy of the object is dropped: its bytes changed. */
+SEXP _bigsnpr_impute(SEXP BM, SEXP method, SEXP ncores) {
+  int n = Rf_asInteger(field(BM, "nrow")), m = Rf_asInteger(field(BM, "ncol")), meth = Rf_asInteger(method), n_all = 0;
+  GetRNGstate();
+  const uint64_t seed = ((uint64_t)(unif_rand() * 4294967296.0) << 32) | (uint64_t)(unif_rand() * 4294967296.0);
+  PutRNGstate();
+  size_t bytes = 0;
+  uint8_t *p = (uint8_t *)fbm_map(BM, 1, 1, &bytes);
+  int rc = bsg_impute(p, n, m, meth, seed, gpu_device(), &n_all);
+  fbm_unmap(p, bytes, 1);
+  Rf_defineVar(Rf_install(".bsg"), R_NilValue, BM);
+  chk(rc);
+  return R_NilValue;
+}
+
 /* _bigsnpr_multLinReg: src/multLinReg.cpp:64-88 (5 arguments; `obj` is a bed or an FBM.code256 environment) */
 SEXP _bigsnpr_multLinReg(SEXP obj, SEXP ind_row, SEXP ind_col, SEXP U, SEXP ncores) {
   bsg_bed *h = any_handle(obj); /* src/multLinReg.cpp:72-78: FBM.code256 or bed, else "Unknown object type." */
@@ -353,8 +391,10 @@ SEXP _bigsnpr_bed_tcrossprod_gpu(SEXP obj_bed, SEXP ind_row, SEXP ind_col, SEXP 
   return K;
 }
 
+/* obj_bed: a bed environment, or an FBM.code256 one with centi-dosage codes and the caller's center / scale (bed_scaleBinom
+ * needs hard calls) */
 SEXP _bigsnpr_bed_randomSVD_gpu(SEXP obj_bed, SEXP ind_row, SEXP ind_col, SEXP center, SEXP scale, SEXP k, SEXP tol) {
-  bsg_bed *h = handle_of(obj_bed);
+  bsg_bed *h = any_handle(obj_bed);
   int nr = LENGTH(ind_row), nc = LENGTH(ind_col), kk = Rf_asInteger(k), niter = 0, nops = 0;
   SEXP d = PROTECT(Rf_allocVector(REALSXP, kk)), u = PROTECT(Rf_allocMatrix(REALSXP, nr, kk));
   SEXP v = PROTECT(Rf_allocMatrix(REALSXP, nc, kk));
@@ -451,6 +491,8 @@ static const R_CallMethodDef CallEntries[] = {
     {"_bigsnpr_writebina", (DL_FUNC)&_bigsnpr_writebina, 5},
     {"_bigsnpr_prod_and_rowSumsSq", (DL_FUNC)&_bigsnpr_prod_and_rowSumsSq, 6},
     {"_bigsnpr_multLinReg", (DL_FUNC)&_bigsnpr_multLinReg, 5},
+    {"_bigsnpr_prod_and_rowSumsSq2", (DL_FUNC)&_bigsnpr_prod_and_rowSumsSq2, 6},
+    {"_bigsnpr_impute", (DL_FUNC)&_bigsnpr_impute, 3},
     {"_bigsnpr_bed_tcrossprod_gpu", (DL_FUNC)&_bigsnpr_bed_tcrossprod_gpu, 5},
     {"_bigsnpr_bed_randomSVD_gpu", (DL_FUNC)&_bigsnpr_bed_randomSVD_gpu, 7},
     {"_bigsnpr_bed_group_gpu", (DL_FUNC)&_bigsnpr_bed_group_gpu, 4},
